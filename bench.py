@@ -2,11 +2,14 @@
 """bench.py — frustums/s forward of the B200 frustum hot path (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
-                    [--workload car|people|sunrgbd] [--batch 32] [--precision 0|1]
+                    [--workload car|people|sunrgbd] [--batch 32] [--precision 0|1] [--dump-outputs DIR]
 
 One "step" = one forward of the hot path (grouping -> PointNet -> FCN -> heads/decode) over one
 batch of `--batch` synthetic frustums per GPU (default: cfgs/det_sample.yaml car, B=32 x 1024
-points = BASELINE.json configs[1]).  Weak scaling: every rank processes its own B frustums;
+points = BASELINE.json configs[1]).  Exactly `--steps` steps are timed per mode (resident, e2e),
+in one region between two CUDA events.  `--dump-outputs DIR` writes what the last timed step
+returned (rank 0) as DIR/<name>.npy; the inputs are seeded, so two builds can be compared
+output for output.  Weak scaling: every rank processes its own B frustums;
 for N>1 the per-rank result block is all-gathered over NCCL inside the timed region (the only
 exchange of the inference path, SURVEY.md section 8(e)).
 
@@ -173,6 +176,26 @@ class _OutRing:
         return v
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+# the 6-tuple PointNetDet.forward returns in eval mode (det_base.py:411)
+OUTPUT_NAMES = ("cls_probs", "center", "heading", "size", "heading_probs", "size_probs")
+
+
+def dump_outputs(path, arrays, seed=0):
+    """Write {name: tensor/array} as path/<name>.npy (float64 stays float64, everything else float32).  Above
+    DUMP_LIMIT_BYTES in all, the same seeded sample of leading-axis rows (frustums) is kept of every array."""
+    arrays = {k: (v.detach().cpu().numpy() if hasattr(v, "detach") else np.asarray(v)) for k, v in arrays.items()}
+    arrays = {k: v if v.dtype == np.float64 else v.astype(np.float32) for k, v in arrays.items()}
+    total = sum(v.nbytes for v in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        n = min(v.shape[0] for v in arrays.values())
+        keep = np.sort(np.random.default_rng(seed).choice(n, max(1, n * DUMP_LIMIT_BYTES // total), replace=False))
+        arrays = {k: v[keep] for k, v in arrays.items()}
+    os.makedirs(path, exist_ok=True)
+    for k, v in arrays.items():
+        np.save(os.path.join(path, k + ".npy"), v)
+
+
 def host_threads():
     """Usable host threads: affinity mask, capped by the cgroup CPU quota when one is set."""
     try:
@@ -323,38 +346,29 @@ def run_train(args, rank, local_rank, world):
         step_e2e(i)
     barrier()
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    counters = {"res": 0, "e2e": 0}
 
-    def region(kind):
-        fn = step_resident if kind == "res" else step_e2e
-        base = counters[kind]
-        counters[kind] += args.steps
+    def region(fn):
+        """Exactly `--steps` steps between two CUDA events -> (ms, what the last step returned)."""
         barrier()
         e0.record()
         for i in range(args.steps):
-            fn(base + i)
+            out = fn(i)
         e1.record()
         barrier()
-        return e0.elapsed_time(e1)
+        return e0.elapsed_time(e1), out
 
-    pilot = torch.tensor([region("res"), region("e2e")], dtype=torch.float64, device=dev)
-    if world > 1:
-        dist.all_reduce(pilot, op=dist.ReduceOp.MAX)
-    R = int(min(max(np.ceil(args.min_seconds * 1e3 / max(float(pilot.min().item()), 1e-3)), 3), args.max_regions))
     sampler = ClockSampler(local_rank)
     if rank == 0:
         sampler.start()
-    t_regions = torch.zeros((2, R), dtype=torch.float64)
-    for r in range(R):
-        t_regions[0, r] = region("res")
-        t_regions[1, r] = region("e2e")
+    t_e2e, _ = region(step_e2e)
+    t_res, (losses, metrics) = region(step_resident)        # last: its final step's results are the dumped outputs
     clocks = sampler.stop() if rank == 0 else None
-    t_regions = t_regions.to(dev)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {**losses, **metrics})
+    t_regions = torch.tensor([t_res, t_e2e], dtype=torch.float64, device=dev)
     if world > 1:
         dist.all_reduce(t_regions, op=dist.ReduceOp.MAX)
-    t_regions = t_regions.cpu().numpy()
-    ms_step = float(np.median(t_regions[0])) / args.steps
-    e2e_ms = float(np.median(t_regions[1])) / args.steps
+    ms_step, e2e_ms = (float(t) / args.steps for t in t_regions.cpu().numpy())
     value, e2e_value = world * B / (ms_step * 1e-3), world * B / (e2e_ms * 1e-3)
     if rank != 0:
         if world > 1:
@@ -422,7 +436,7 @@ def run_train(args, rank, local_rank, world):
                                  "overlapping the PointNet backward" % (ts.flat.numel * 4 / 1e6),
                    "l2": "inputs cycle through a %d-batch pool; every step rewrites ~0.4 GB of activations / "
                          "gradients (> 126 MB L2)" % npool,
-                   "timing": "median of %d repeated %d-step regions (resident and e2e regions alternate)" % (R, args.steps)},
+                   "timing": "one %d-step region per mode (e2e, then resident)" % args.steps},
         "e2e": {"value": e2e_value, "unit": UNIT, "h2d_bytes_per_step": h2d_bytes, "d2h_bytes_per_step": 4},
         "gpu_launches": eng.kernel_launches_per_step() * args.steps,
         "launches_per_step": eng.kernel_launches_per_step(),
@@ -461,12 +475,15 @@ def main():
     ap.add_argument("--exchange", default="peer", choices=["peer", "nccl"],
                     help="N>1 result exchange: peer = the heads epilogue stores every rank's rows into all ranks' "
                          "gather buffers over NVLink (no collective); nccl = all_gather_into_tensor per step")
-    ap.add_argument("--min-seconds", type=float, default=0.5,
-                    help="device time to accumulate per mode by repeating the K-step region (median reported)")
-    ap.add_argument("--max-regions", type=int, default=400)
     ap.add_argument("--streams", type=int, default=int(os.environ.get("FCN_STREAMS", "10")),
                     help="forwards in flight: steps are issued round-robin on this many CUDA streams")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step returned as DIR/<name>.npy (float32/float64, <= 64 MB)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs times the GPU path; --impl reference has no GPU outputs")
+    if args.steps < 1:
+        ap.error("--steps must be >= 1")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -663,52 +680,40 @@ def main():
         step_e2e(i, last=(i == nwarm - 1))
     barrier()
 
-    # ---- timed regions.  ONE region = EXACTLY `--steps` steps between two CUDA events, barrier + synchronize on
-    # both sides.  A 20-step region lasts only ~3 ms, so the region is REPEATED R times (R chosen so that each
-    # mode accumulates >= ~0.5 s of device time, bounded) and the MEDIAN region is reported; resident and e2e
-    # regions ALTERNATE, so both medians see the same clocks / thermal state.  Per region the max over ranks is
-    # taken (one all-reduce over the vector of region times after the loop).
+    # ---- timed regions.  ONE region per mode = EXACTLY `--steps` steps between two CUDA events, barrier +
+    # synchronize on both sides; the max over ranks is taken.  The e2e region runs first, so that the last timed
+    # step is a resident one: `value` is measured on that path and its last step's results are the dumped outputs.
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    counters = {"res": 0, "e2e": 0}
 
-    def region(kind):
-        fn = step_resident if kind == "res" else step_e2e
-        base = args.warmup + counters[kind]
-        counters[kind] += args.steps
+    def region(fn):
         barrier()
         e0.record()
         fork_streams()
         for i in range(args.steps):
-            fn(base + i, last=(i == args.steps - 1))
+            out = fn(args.warmup + i, last=(i == args.steps - 1))
         join_streams()
         e1.record()
         barrier()
-        return e0.elapsed_time(e1)
+        return e0.elapsed_time(e1), out
 
-    pilot = torch.tensor([region("res"), region("e2e")], dtype=torch.float64, device=dev)
-    if world > 1:
-        dist.all_reduce(pilot, op=dist.ReduceOp.MAX)
-    R = int(min(max(np.ceil(args.min_seconds * 1e3 / max(float(pilot.min().item()), 1e-3)), 3), args.max_regions))
     sampler = ClockSampler(local_rank)
     if rank == 0:
         sampler.start()
-    t_regions = torch.zeros((2, R), dtype=torch.float64)
-    for r in range(R):
-        t_regions[0, r] = region("res")
-        t_regions[1, r] = region("e2e")
-    clocks = sampler.stop() if rank == 0 else None    # samples cover all timed regions (resident + e2e)
-    t_regions = t_regions.to(dev)
+    t_e2e, _ = region(step_e2e)
+    t_res, last_out = region(step_resident)
+    clocks = sampler.stop() if rank == 0 else None    # samples cover both timed regions
+    if args.dump_outputs and rank == 0:   # before any later step overwrites the plan's output block
+        dump_outputs(args.dump_outputs, dict(zip(OUTPUT_NAMES, last_out)))
+    t_regions = torch.tensor([t_res, t_e2e], dtype=torch.float64, device=dev)
     if world > 1:
         dist.all_reduce(t_regions, op=dist.ReduceOp.MAX)
     t_regions = t_regions.cpu().numpy()
-    ms_total = float(np.median(t_regions[0]))
-    ms_step = ms_total / args.steps
+    ms_step = float(t_regions[0]) / args.steps
     value = world * B / (ms_step * 1e-3)
-    e2e_ms_step = float(np.median(t_regions[1])) / args.steps
+    e2e_ms_step = float(t_regions[1]) / args.steps
     e2e_value = world * B / (e2e_ms_step * 1e-3)
-    spread = {"regions": R, "steps_per_region": args.steps,
-              "resident_ms_per_step_p10_p50_p90": [float(np.percentile(t_regions[0], q)) / args.steps for q in (10, 50, 90)],
-              "e2e_ms_per_step_p10_p50_p90": [float(np.percentile(t_regions[1], q)) / args.steps for q in (10, 50, 90)],
+    spread = {"regions": 1, "steps_per_region": args.steps,
+              "resident_ms_per_step": ms_step, "e2e_ms_per_step": e2e_ms_step,
               "device_seconds_timed": float(t_regions.sum() * 1e-3),
               "e2e_le_value": bool(e2e_value <= value * 1.02)}
 
@@ -800,7 +805,7 @@ def main():
             "l2": "inputs cycle through a %d-batch pool (%.0f MB > 126 MB L2); weights/workspaces stay L2-resident"
                   % (npool, npool * step_in_bytes / 1e6),
             "cuda_graph": True, "precision": roofline["precision"], "streams_in_flight": nstream,
-            "timing": "median of %d repeated %d-step regions (resident and e2e regions alternate)" % (spread["regions"], args.steps),
+            "timing": "one %d-step region per mode (e2e, then resident)" % args.steps,
             "collective": ("none (single GPU)" if world == 1 else
                            "none: the heads epilogue of every forward stores its %d KB result block into all %d ranks' "
                            "gather buffers over NVLink peer memory (CUDA IPC) + one epoch flag per forward"

@@ -8,9 +8,21 @@ from conftest import GOLDEN_CASES, load_golden
 from oracle import model as om
 from oracle import qdp
 
+# The fixtures were written by torch on the CPU with 8 intra-op threads.  oneDNN splits convolution reductions by
+# thread count, so the fp32 sums only round the same way with the same count, whatever the host's core count.
+GOLDEN_THREADS = 8
+
+
+@pytest.fixture
+def golden_threads():
+    n = torch.get_num_threads()
+    torch.set_num_threads(GOLDEN_THREADS)
+    yield
+    torch.set_num_threads(n)
+
 
 @pytest.mark.parametrize("name", list(GOLDEN_CASES))
-def test_oracle_model_matches_reference_golden(name):
+def test_oracle_model_matches_reference_golden(name, golden_threads):
     g, data, sd, w, cfg = load_golden(name)
     arch = w["arch"]
     from frustum_convnet_b200.config import DATASET_INFO
