@@ -187,8 +187,10 @@ SIGNATURES = {
     "fcn_train_pool": (_I, [C.POINTER(TrainPool), _I, _P]),
     "fcn_train_finalize": (_I, [_P, _I, _I, _P]),
     "fcn_adam_step": (_I, [_P, _P, _P, _P, C.c_longlong, _F, _F, _F, _F, _F, _I, _F, _P]),
-    "fcn_rotate_nms_3d": (_I, [_I, _P, _P, _F, _I, _P, _P, _I, _P]),
+    "fcn_rotate_nms_3d": (_I, [_I, _P, _P, _I, _F, _I, _P, _P, _I, _P, C.c_longlong, _P]),
+    "fcn_rotate_nms_3d_workspace_bytes": (C.c_longlong, [_I, _I]),
     "fcn_rotate_nms_3d_max_dets": (_I, []),
+    "fcn_rotate_nms_3d_max_seg_len": (_I, []),
     "fcn_det_loss": (_I, [C.POINTER(LossArgs), _P]),
     "fcn_build_inputs": (_I, [C.POINTER(InputArgs), _P]),
     "fcn_ipc_export": (_I, [_P, _P, C.POINTER(C.c_longlong)]),

@@ -356,14 +356,25 @@ FCN_API int fcn_det_loss(const fcn_loss_args *args, fcn_stream_t stream);
  *     `cube_nms` = rotate_nms_3d_cc (ops/pybind11/rbbox_iou.py:294-311) -> rotate_non_max_suppression_3d_cpu
  *     (ops/pybind11/nms_cpu.h:148-240), called per image and class from train/test_net_det.py:126-152.
  *     dets: (total, 8) fp32 rows [cx, cy, cz, l, w, h, ry, score]; segment s = rows
- *     [seg_offsets[s], seg_offsets[s+1]) (one image x class list, at most fcn_rotate_nms_3d_max_dets() rows are
- *     considered); keep: (num_segments, keep_stride) int32 GLOBAL row indices in descending-score order,
- *     keep_count[s] <= top_k of them are valid.  A box is suppressed by a kept, higher-scored box when their
- *     axis-aligned bounding cubes overlap and the rotated 3-D IoU is >= thresh.
+ *     [seg_offsets[s], seg_offsets[s+1]) (one image x class list; every row of it is considered, no list is
+ *     truncated); keep: (num_segments, keep_stride) int32 GLOBAL row indices in descending-score order,
+ *     keep_count[s] <= top_k <= keep_stride of them are valid.  A box is suppressed by a kept, higher-scored box
+ *     when their axis-aligned bounding cubes overlap and the rotated 3-D IoU is >= thresh.  Score order: NaN
+ *     first, then descending score, equal scores (and NaNs) larger index first = np.argsort(kind="stable")[::-1].
+ *     A box with NaN geometry is never suppressed and suppresses nothing.
+ *     max_seg_len: an upper bound of every segment length (<= fcn_rotate_nms_3d_max_seg_len()).  Segments of at
+ *     most fcn_rotate_nms_3d_max_dets() rows run in shared memory, one launch in all; longer ones need `workspace`
+ *     (256-byte aligned, device memory) of fcn_rotate_nms_3d_workspace_bytes(number of longer segments,
+ *     max_seg_len) bytes, NULL otherwise.  A segment longer than max_seg_len, with a negative length, or left
+ *     without a workspace slot gets keep_count[s] = -1 (an error for the caller to raise).  Returns an error,
+ *     before any CUDA call, for top_k > keep_stride, a negative max_seg_len or a missing / too small workspace.
  * ------------------------------------------------------------------------------------------ */
-FCN_API int fcn_rotate_nms_3d(int num_segments, const float *dets, const int32_t *seg_offsets, float thresh, int top_k,
-                              int32_t *keep, int32_t *keep_count, int keep_stride, fcn_stream_t stream);
+FCN_API int fcn_rotate_nms_3d(int num_segments, const float *dets, const int32_t *seg_offsets, int max_seg_len,
+                              float thresh, int top_k, int32_t *keep, int32_t *keep_count, int keep_stride,
+                              void *workspace, long long workspace_bytes, fcn_stream_t stream);
+FCN_API long long fcn_rotate_nms_3d_workspace_bytes(int num_long_segments, int max_seg_len);
 FCN_API int fcn_rotate_nms_3d_max_dets(void);
+FCN_API int fcn_rotate_nms_3d_max_seg_len(void);
 
 /* ------------------------------------------------------------------------------------------
  * (9) Device-side input builder ("next" row 8(f)-3): ProviderDataset.__getitem__ of datasets/provider_sample.py

@@ -11,11 +11,14 @@ models/det_base.py:494-503 on the corners of models/model_util.py:48-72):
   * out[n] = (inter_area / union_area, inter_vol / (vol + qvol - inter_vol)); pairs without intersection keep
     the zero initialisation (box_ops.h:199,226,247-248); N != K or N == 0 returns zeros (box_ops.h:201-203).
 
-PARITY UNPINNED for the polygon clipping itself: the reference delegates it to Boost.Geometry (unversioned
-system dependency, absent from /root/reference and from this image).  This file restates the published
-algorithm for two CONVEX polygons (Sutherland-Hodgman clipping + shoelace area; the union of two overlapping
-convex polygons is one polygon of area a + b - inter) in float64 and is cross-checked in
-tests/test_box_iou_cpu.py against closed-form cases and an independent point-sampling estimate.
+PINNED to the reference's Python IoU for convex, non-degenerate boxes.  The reference delegates the polygon
+clipping to Boost.Geometry (an unversioned system dependency, not available here), but it also ships the same
+metric in pure Python, utils/box_util.py (polygon_clip + ConvexHull; models/det_base.py:28).  This file restates
+the published algorithm for two CONVEX polygons (Sutherland-Hodgman clipping + shoelace area; the union of two
+overlapping convex polygons is one polygon of area a + b - inter) in float64; tests/test_box_iou_cpu.py checks it
+against tests/golden/iou_ref.npz, box_util's values on ~2 200 pairs in named groups written by
+oracle/make_golden_iou.py (BEV to 1e-9; 3-D to 4e-6, the gap between box_util's edge-length volume and Boost's
+area * height on float32 corners), and against closed-form cases and an independent point-sampling estimate.
 
 DEGENERATE RINGS (decision of round 2, pinned by tests/test_box_iou_cpu.py::test_degenerate_boxes): the reference
 appends the four BEV corners without `bg::correct` (box_ops.h:206-224).  A decoded box with exactly ONE negative

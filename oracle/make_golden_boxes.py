@@ -3,7 +3,8 @@
 Runs the UNMODIFIED reference `get_box3d_corners_helper` (models/model_util.py:48-72) on seeded box pairs
 (prediction = perturbed ground truth, the situation of models/det_base.py:488-495) and stores inputs + corners
 as tests/golden/box_pairs.npz.  The IoU values themselves cannot come from the reference here (Boost.Geometry
-is absent: `parity unpinned`, see oracle/box_iou.py); the fixture pins the corner convention the IoU consumes.
+is absent; oracle/make_golden_iou.py takes them from the reference's Python IoU instead); the fixture pins the
+corner convention the IoU consumes.
 
     python -m oracle.make_golden_boxes          # authoring container only (needs /root/reference)
 """

@@ -48,6 +48,29 @@ def test_argument_validation_without_gpu():
     assert lib.fcn_rbbox_iou_3d_pair(1, base + 4, base, base, 0.5, None, None) == -1
     assert b"aligned" in lib.fcn_last_error()
     assert lib.fcn_rbbox_iou_3d_pair(0, None, None, None, 0.5, None, None) == 0   # nothing to do, no stats
+    # rotated 3-D NMS: sizes, keep-row overflow and the long-list workspace are checked before any CUDA call
+    nms = lib.fcn_rotate_nms_3d
+    p = buf.ctypes.data
+    assert nms(1, p, p, 10, 0.5, 300, p, p, 299, None, 0, None) == -1            # top_k > keep_stride
+    assert b"keep_stride" in lib.fcn_last_error()
+    assert nms(0, None, None, 0, 0.5, 8, None, None, 4, None, 0, None) == -1      # ... even with no segment
+    assert nms(1, p, p, -1, 0.5, 8, p, p, 8, None, 0, None) == -1                # negative length
+    assert b"max_seg_len" in lib.fcn_last_error()
+    assert nms(1, p, p, 513, 0.5, 8, p, p, 8, None, 0, None) == -1               # long list, no workspace
+    assert b"workspace" in lib.fcn_last_error()
+    need = lib.fcn_rotate_nms_3d_workspace_bytes(1, 2000)
+    assert need >= 2000 * (2000 // 32) * 4                                       # holds the n x n/32 bit matrix
+    assert nms(1, p, p, 2000, 0.5, 8, p, p, 8, base, need - 1, None) == -1        # too small
+    assert nms(1, p, p, 2000, 0.5, 8, p, p, 8, base + 4, need, None) == -1        # misaligned
+    assert b"aligned" in lib.fcn_last_error()
+    assert nms(1, None, p, 10, 0.5, 8, p, p, 8, None, 0, None) == -1             # NULL
+    assert nms(0, None, None, 0, 0.5, 8, None, None, 8, None, 0, None) == 0       # nothing to do
+    ws = lib.fcn_rotate_nms_3d_workspace_bytes
+    assert ws(0, 2000) == 0 and ws(5, 512) == 0 and ws(3, 513) > 0
+    assert ws(2, 2000) > ws(1, 2000) and ws(1, 4000) > 3 * ws(1, 2000)
+    assert ws(-1, 600) == -1 and ws(1, -5) == -1
+    assert ws(1, lib.fcn_rotate_nms_3d_max_seg_len() + 1) == -1
+    assert lib.fcn_rotate_nms_3d_max_dets() == 512
 
 
 def test_box_iou_wrapper_rejects_cpu_tensors_and_bad_shapes():

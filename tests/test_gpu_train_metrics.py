@@ -1,6 +1,7 @@
 """GPU: pairwise rotated-box IoU of the train metrics (SURVEY.md 8(f)-1) through the C ABI against the oracle
-(oracle/box_iou.py; Boost.Geometry is absent, so the clipping itself is parity-unpinned - see its header).
-Tolerance: 1e-4 absolute on IoU values in [0, 1] (fp32 kernel with FMA contraction vs float64 oracle)."""
+(oracle/box_iou.py) and against the reference's own Python IoU (utils/box_util.py, held in
+tests/golden/iou_ref.npz): pinned to the reference for convex, non-degenerate boxes.
+Tolerance: 1e-4 absolute on IoU values in [0, 1] (fp32 kernel with FMA contraction vs float64 values)."""
 import os
 
 import numpy as np
@@ -34,6 +35,25 @@ def test_iou_matches_oracle_on_reference_generated_corners():
     hi = (want[:, 1] >= 0.7 - 1e-3).mean()
     assert lo - 1e-6 <= float(frac) <= hi + 1e-6
     assert torch.equal(rbbox_iou_3d_pair(pr, gt), out)                     # without stats: same values
+
+
+def test_iou_matches_reference_python_iou():
+    """fcn_rbbox_iou_3d_pair on every group of the reference-held fixture, incl. the two mean statistics."""
+    from frustum_convnet_b200.box_iou import rbbox_iou_3d_pair
+    g = dict(np.load(os.path.join(GOLDEN_DIR, "iou_ref.npz")))
+    want = g["iou"]
+    pr, gt = torch.from_numpy(g["pr_corners"]).cuda(), torch.from_numpy(g["gt_corners"]).cuda()
+    out, (m2, m3, frac) = rbbox_iou_3d_pair(pr, gt, iou_thresh=0.5)
+    got = out.cpu().numpy()
+    err = np.abs(got - want)
+    print("device vs reference IoU: worst BEV %.2e, 3-D %.2e; means %.2e %.2e" % (
+        *err.max(0), abs(float(m2) - want[:, 0].mean()), abs(float(m3) - want[:, 1].mean())))
+    assert np.isfinite(got).all() and err.max() <= TOL
+    for k, name in enumerate(g["group_names"]):
+        assert err[g["group"] == k].max() <= TOL, name
+    assert abs(float(m2) - want[:, 0].mean()) <= TOL and abs(float(m3) - want[:, 1].mean()) <= TOL
+    lo, hi = (want[:, 1] >= 0.5 + 1e-3).mean(), (want[:, 1] >= 0.5 - 1e-3).mean()
+    assert lo - 1e-6 <= float(frac) <= hi + 1e-6
 
 
 def test_iou_edge_cases_and_scale():
